@@ -4,7 +4,7 @@
 preprocess -> ICP -> raycast -> k-NN/DQB warp -> data-term solve -> warp -> project/remove -> integrate -> extract ->
 raycast loop on one B200).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one frame.  N > 1 (under torchrun, one rank per GPU): every rank runs an independent sequence (seed = rank,
 config 5): weak scaling, no data-path collective; timing is the max over ranks.
@@ -257,6 +257,37 @@ def integrate_kernel_name():
     return {5: "integrate_kernel_v5", 3: "integrate_kernel_v3"}.get(code, "integrate_kernel<4>")
 
 
+def dump_outputs(k, out_dir: Path, max_points: int = 1 << 20, volume_samples: int = 1 << 20):
+    """what the last timed frame left for a caller of the frame loop, as DIR/<name>.npy (float32, under 64 MB in all): the camera
+    pose [R | t], the ray-cast point / normal maps, the warp nodes, the canonical cloud and its normals (rows sorted by their bit
+    patterns, since extraction appends in no fixed order; a seeded sample of `max_points` rows if larger) and a seeded sample of
+    `volume_samples` voxels of the TSDF (value and weight).  The ray-cast maps and the cloud normals mark "no hit" / "no normal"
+    with NaN: they are written with 0 in place of every non-finite value, and <name>_valid.npy holds 1 for each row (pixel, point)
+    whose values are all finite, 0 otherwise.  Same arguments, same inputs, same sample: two builds compare output for output."""
+    out_dir.mkdir(parents=True, exist_ok=True)
+    R, t = k.getCameraPose()
+    arrays = {"camera_pose": np.concatenate([R, t[:, None]], axis=1), "raycast_points": k.buffer("prev_points"),
+              "raycast_normals": k.buffer("prev_normals"), "warp_nodes": k.buffer("nodes")[: k.info()["nodes"]]}
+    cloud, normals = k.buffer("cloud"), k.buffer("cloud_normals")
+    order = np.lexsort(np.ascontiguousarray(cloud).view(np.uint32).T[::-1])
+    if len(order) > max_points:
+        order = order[np.sort(np.random.default_rng(0).choice(len(order), max_points, replace=False))]
+    arrays["cloud_points"], arrays["cloud_normals"] = cloud[order], normals[order]
+    vol = k.buffer("volume")
+    vox = np.sort(np.random.default_rng(1).integers(0, vol.size, volume_samples))
+    arrays["volume_tsdf_sample"] = (vol[vox] & 0xFFFF).astype(np.uint16).view(np.float16).astype(np.float32)
+    arrays["volume_weight_sample"] = (vol[vox] >> 16).astype(np.float32)
+    for name in ("raycast_points", "raycast_normals", "cloud_normals"):
+        finite = np.isfinite(arrays[name])
+        arrays[f"{name}_valid"] = finite.all(axis=-1)
+        arrays[name] = np.where(finite, arrays[name], np.float32(0))
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, np.float32)
+        if not np.isfinite(a).all():
+            raise ValueError(f"--dump-outputs: {name} holds non-finite values")
+        np.save(out_dir / f"{name}.npy", a)
+
+
 def bench_config(world: int, first: int, K: int):
     """the SAME dict in both arms (the driver compares them): workload + the timed window, nothing measured"""
     return {"workload": WORKLOAD, "node_cap": MAX_NODES, "knn": 8, "solver": "LM 5 x PCG 100 (early-out)", "sequences": world,
@@ -359,6 +390,8 @@ def main():
     ap.add_argument("--frames-from", type=int, default=10, help="first TIMED frame of the sequence (SURVEY 8d: steady state = frames 10-99): frame 0 "
                     "initialises, frames 1..F-1 are untimed (the last W of them are the warm-up steps), frames F..F+K-1 are timed")
     ap.add_argument("--no-traffic-probe", action="store_true", help="do not run the one-launch ncu pass that measures the integrate / ray-cast DRAM bytes")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path, help="write what the last timed frame computed (device-resident arm, rank 0) "
+                    "as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 
@@ -398,7 +431,7 @@ def main():
         p.flags = flags
         return p
 
-    def timed(run_frame):
+    def timed(run_frame, dump_dir=None):
         """frame 0 + the untimed frames 1..first-1 (the last W = warm-up), then exactly K frames between barrier+sync, CUDA events on the
         launching stream (one event per frame: the whole-region time is ev[0] -> ev[K], the per-frame spread comes for free)"""
         sampler = ClockSampler(local_rank)
@@ -425,13 +458,16 @@ def main():
         info = k.info()
         Rf, tf = k.getCameraPose()
         digest = {"digest": k.state_digest(), "pose": [float(x) for x in Rf.reshape(9)] + [float(x) for x in tf]}
+        if dump_dir is not None and rank == 0:
+            dump_outputs(k, dump_dir)
         k.close()
         ms, _total, ok = distrib.aggregate(ms, ok, device)       # max time over ranks; ok = fewest fused frames on any rank
         return ms, ok, info, clocks, per, digest
 
     pitch = COLS * 2
     # value: inputs already resident in HBM
-    ms_dev, ok_dev, info, clocks, per_dev, digest_dev = timed(lambda k, t: k.lib.df_kinfu_process_device(k.h, frames_dev[t].data_ptr(), pitch))
+    ms_dev, ok_dev, info, clocks, per_dev, digest_dev = timed(lambda k, t: k.lib.df_kinfu_process_device(k.h, frames_dev[t].data_ptr(), pitch),
+                                                              args.dump_outputs)
     # e2e: the reference-facing call with HOST buffers (pinned), H2D + D2H inside the timed region
     ms_e2e, ok_e2e, _, clocks_e2e, per_e2e, digest_e2e = timed(lambda k, t: k.lib.df_kinfu_process_host(k.h, frames_pinned[t].data_ptr(), pitch))
     assert ok_dev == K and ok_e2e == K, f"tracking was lost during the timed region ({ok_dev}/{ok_e2e} of {K} frames fused)"

@@ -100,69 +100,6 @@ def build_cpp_program(src: Path, out: Path) -> Path:
     return out
 
 
-REF_DEMO_SRC = Path("/root/reference/apps/demo.cpp")
-REF_DEMO_BIN = ROOT / "tests" / "cpp" / "_build" / "ref_demo"
-
-
-def build_reference_demo(force: bool = False):
-    """The reference's OWN apps/demo.cpp, compiled from where it lies and UNCHANGED, against include/kfusion + the headless OpenCV
-    stand-ins (include/cvcompat) and linked with libkfusion.so / libdfusion.so -- the drop-in claim of INTEGRATION.md made literal.
-    Only possible where /root/reference exists; the binary (git-ignored) travels to the GPU box with the snapshot."""
-    if not REF_DEMO_SRC.exists():
-        return None
-    build_mirror()
-    REF_DEMO_BIN.parent.mkdir(parents=True, exist_ok=True)
-    deps = [REF_DEMO_SRC, MIRROR_LIB] + sorted((ROOT / "include").rglob("*.h*"))
-    if not force and REF_DEMO_BIN.exists() and all(d.stat().st_mtime <= REF_DEMO_BIN.stat().st_mtime for d in deps):
-        return REF_DEMO_BIN
-    gxx = "/usr/bin/g++" if Path("/usr/bin/g++").exists() else "g++"
-    cmd = [gxx, "-std=c++17", "-O1", "-w", *MIRROR_INC, "-o", str(REF_DEMO_BIN), str(REF_DEMO_SRC), "-L", str(HERE), "-lkfusion", "-ldfusion",
-           "-lz", "-Wl,-rpath," + str(HERE), "-Wl,-rpath,$ORIGIN/../../../dynamicfusion_b200"]
-    r = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
-    if r.returncode != 0:
-        raise RuntimeError("building the reference's apps/demo.cpp failed:\n" + r.stdout)
-    return REF_DEMO_BIN
-
-
-REF_TESTS_DIR = Path("/root/reference/tests")
-REFCOMPAT = ROOT / "tests" / "cpp" / "refcompat"
-
-
-def build_reference_tests(force: bool = False) -> dict:
-    """The reference's OWN test files (tests/warp_test.cpp, tests/utils/test_{quaternion,dual_quaternion}.cc), compiled unchanged
-    from where they lie with a minimal GoogleTest stand-in (tests/cpp/refcompat/gtest/gtest.h):
-      mine_*  against this repo's headers (include/) -- warp_test also links libkfusion.so and needs a GPU to run;
-      ref_*   the two header-only quaternion tests against the REFERENCE's own headers (oracle/ref_shim supplies cv::Vec3f).
-    Returns {name: path}; empty where /root/reference is absent.  Binaries are git-ignored and travel to the GPU box."""
-    if not REF_TESTS_DIR.exists():
-        return {}
-    build_mirror()
-    out_dir = ROOT / "tests" / "cpp" / "_build"
-    out_dir.mkdir(parents=True, exist_ok=True)
-    gxx = "/usr/bin/g++" if Path("/usr/bin/g++").exists() else "g++"
-    main_cpp = str(REFCOMPAT / "gtest_main.cpp")
-    jobs = {}
-    for t in ("test_quaternion", "test_dual_quaternion"):
-        src = str(REF_TESTS_DIR / "utils" / f"{t}.cc")
-        jobs[f"mine_{t}"] = [gxx, "-std=c++17", "-O1", "-w", "-ffp-contract=off", "-I", str(REFCOMPAT), *MIRROR_INC, src, main_cpp]
-        jobs[f"ref_{t}"] = [gxx, "-std=c++11", "-O1", "-w", "-ffp-contract=off", "-I", str(REFCOMPAT), "-I", str(ROOT / "oracle" / "ref_shim"),
-                            "-I", "/root/reference/kfusion/include", "-I", "/root/reference/kfusion/src/utils", src, main_cpp]
-    jobs["mine_warp_test"] = [gxx, "-std=c++17", "-O1", "-w", "-I", str(REFCOMPAT), *MIRROR_INC, "-I", str(ROOT / "include" / "opt"),
-                              str(REF_TESTS_DIR / "warp_test.cpp"), main_cpp, "-L", str(HERE), "-lkfusion", "-ldfusion",
-                              "-Wl,-rpath," + str(HERE), "-Wl,-rpath,$ORIGIN/../../../dynamicfusion_b200"]
-    jobs["mine_ceres_warp_test"] = [gxx, "-std=c++17", "-O1", "-w", "-I", str(REFCOMPAT), *MIRROR_INC, str(REF_TESTS_DIR / "ceres_warp_test.cpp"), main_cpp,
-                                    "-L", str(HERE), "-lkfusion", "-ldfusion", "-Wl,-rpath," + str(HERE), "-Wl,-rpath,$ORIGIN/../../../dynamicfusion_b200"]
-    built = {}
-    for name, cmd in jobs.items():
-        exe = out_dir / name
-        if force or not exe.exists() or exe.stat().st_mtime < MIRROR_LIB.stat().st_mtime:
-            r = subprocess.run(cmd + ["-o", str(exe)], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
-            if r.returncode != 0:
-                raise RuntimeError(f"building the reference's {name} failed:\n" + r.stdout)
-        built[name] = exe
-    return built
-
-
 if __name__ == "__main__":
     print(build(force="--force" in sys.argv, verbose="-v" in sys.argv))
     if "--mirror" in sys.argv:

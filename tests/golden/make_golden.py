@@ -5,6 +5,7 @@
 Needs oracle/_ref/{knn_ref,dq_ref} (built by `make -C oracle ref` from /root/reference: the vendored nanoflann + the
 reference's knn_point_cloud.hpp / quaternion.hpp / dual_quaternion.hpp, compiled as they lie).  Writes
 tests/golden/knn_ref.json and tests/golden/dq_ref.json; floats are stored as C99 hex strings so they round-trip exactly.
+tests/golden/knn_ref_random.npz holds the reference's 8-NN of the random clouds of tests/test_oracle_golden.py.
 /root/reference does not exist on the GPU box, so the committed JSON files are what the tests read there."""
 import json
 import subprocess
@@ -36,6 +37,18 @@ def knn():
     (HERE / "knn_ref.json").write_text(json.dumps({"source": "reference nanoflann + knn_point_cloud.hpp via oracle/ref_shim/knn_ref.cpp", "cases": cases}))
 
 
+def knn_random():
+    """the seeded clouds of tests/test_oracle_golden.py::test_knn_matches_reference_nanoflann_binary"""
+    rng = np.random.default_rng(5)
+    pts = rng.uniform(-1, 1, (300, 3)).astype(np.float32)
+    qs = rng.uniform(-1.2, 1.2, (200, 3)).astype(np.float32)
+    inp = f"{len(pts)} {len(qs)}\n" + "\n".join(" ".join(repr(float(v)) for v in p) for p in np.vstack([pts, qs]))
+    out = subprocess.run([str(REF / "knn_ref")], input=inp, capture_output=True, text=True, check=True).stdout.split()
+    idx = np.array(out[0::2], np.int16).reshape(len(qs), 8)
+    d2 = np.array([np.float32(float.fromhex(v)) for v in out[1::2]], np.float32).reshape(len(qs), 8)
+    np.savez_compressed(HERE / "knn_ref_random.npz", idx=idx, d2=d2)
+
+
 def dq():
     rng = np.random.default_rng(7)
     K = 150
@@ -63,5 +76,6 @@ def dq():
 
 if __name__ == "__main__":
     knn()
+    knn_random()
     dq()
-    print("wrote", HERE / "knn_ref.json", HERE / "dq_ref.json")
+    print("wrote", HERE / "knn_ref.json", HERE / "knn_ref_random.npz", HERE / "dq_ref.json")

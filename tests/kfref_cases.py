@@ -120,6 +120,26 @@ def all_cases(orc, ref):
     return {f"{c}/{k}": v for c, d in cases.items() for k, v in d.items()}
 
 
+def render_scene(orc):
+    """inputs of the display kernels (tests/test_render_gpu.py): the 128^3 umbrella volume integrated from the identity pose, its
+    ray-cast point / normal maps, and the depth frame with a hole of the depth-path image ops.  Poses are formed as
+    host.TsdfVolume.integrate / raycast form them, so the volume equals the GPU's bit for bit."""
+    from dynamicfusion_b200 import host
+    dim = 128
+    dims, vs = (dim,) * 3, (1.0 / dim,) * 3
+    vol_pose, pose = synth.volume_pose(1.0), host.identity_pose()
+    vol = np.zeros(dim ** 3, np.uint32)
+    orc.clear_volume(vol, dims, vs, TRUNC, MAXW)
+    orc.integrate(vol, dims, vs, TRUNC, MAXW, orc.compute_dists(synth.umbrella_depth(0), K), host.aff_mul(host.aff_inv(pose), vol_pose), K)
+    cam2vol = host.aff_mul(host.aff_inv(vol_pose), pose)
+    Rinv = np.linalg.inv(cam2vol[0].astype(np.float64)).astype(np.float32)
+    pts, nrm, _ = orc.raycast_points(vol, dims, vs, TRUNC, MAXW, cam2vol, Rinv, K, 640, 480, 0.75, 0.5)
+    depth = synth.umbrella_depth(2)
+    depth[100:140, 200:260] = 0                                              # a hole
+    return {"dims": dims, "voxel_size": vs, "volume": vol, "cam2vol": cam2vol, "Rinv": Rinv, "points": np.ascontiguousarray(pts),
+            "normals": np.ascontiguousarray(nrm), "depth": depth}
+
+
 def canonical_bytes(a: np.ndarray) -> bytes:
     """bit pattern with every NaN mapped to one quiet NaN (payloads are not part of the contract)"""
     a = np.ascontiguousarray(a)

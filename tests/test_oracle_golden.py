@@ -99,20 +99,15 @@ def test_knn_orders_match_nanoflann(orc):
 
 
 def test_knn_matches_reference_nanoflann_binary(orc):
-    """when oracle/_ref/knn_ref (the reference's vendored nanoflann + knn_point_cloud.hpp compiled as they lie) was built,
-    compare on random clouds: squared distances bit-exact, index lists equal wherever distances are distinct"""
-    import subprocess
+    """against what oracle/_ref/knn_ref (the reference's vendored nanoflann + knn_point_cloud.hpp compiled as they lie) returned
+    for these random clouds (tests/golden/knn_ref_random.npz, written by tests/golden/make_golden.py): squared distances
+    bit-exact, index lists equal wherever distances are distinct"""
     from pathlib import Path
-    exe = Path(orc.HERE) / "_ref" / "knn_ref"
-    if not exe.exists():
-        pytest.skip("oracle/_ref/knn_ref not built (needs /root/reference)")
     rng = np.random.default_rng(5)
     pts = rng.uniform(-1, 1, (300, 3)).astype(np.float32)
     qs = rng.uniform(-1.2, 1.2, (200, 3)).astype(np.float32)
-    inp = f"{len(pts)} {len(qs)}\n" + "\n".join(" ".join(repr(float(v)) for v in p) for p in np.vstack([pts, qs]))
-    out = subprocess.run([str(exe)], input=inp, capture_output=True, text=True, check=True).stdout.split()
-    ref_idx = np.array(out[0::2], np.int64).reshape(len(qs), 8)
-    ref_d2 = np.array([np.float32(float.fromhex(v)) for v in out[1::2]], np.float32).reshape(len(qs), 8)
+    golden = np.load(Path(__file__).parent / "golden" / "knn_ref_random.npz")
+    ref_idx, ref_d2 = golden["idx"].astype(np.int64), golden["d2"]
     idx, d2 = orc.knn8(orc.make_nodes(pts), qs)
     assert np.array_equal(d2.view(np.uint32), ref_d2.view(np.uint32))
     distinct = np.ones(len(qs), bool)
