@@ -77,6 +77,8 @@ PROTOTYPES = {
     "df_extract_cloud": (_i, [Volume, Aff3f, _vp, _i, _vp, _vp, _vp]),
     "df_extract_cloud_tracked": (_i, [Volume, Aff3f, _vp, _i, _vp, _vp, _vp, _vp]),
     "df_extract_normals": (_i, [Volume, _vp, _i, _vp, Aff3f, C.POINTER(C.c_float), _f, _vp, _vp]),
+    "df_extract_mesh_workspace_bytes": (_sz, [Volume]),
+    "df_extract_mesh": (_i, [Volume, Aff3f, _vp, _vp, _vp, _i, _vp, _i, _vp, _vp, _vp]),
     "df_bilateral": (_i, [_vp, _sz, _i, _i, _vp, _sz, _i, _f, _f, _vp]),
     "df_truncate_depth": (_i, [_vp, _sz, _i, _i, _f, _vp]),
     "df_pyr_down": (_i, [_vp, _sz, _i, _i, _vp, _sz, _f, _vp]),
@@ -126,6 +128,7 @@ PROTOTYPES = {
     "df_kinfu_join": (_i, [_vp]),
     "df_kinfu_set_overrides": (_i, [_vp, _vp, _sz, _vp, _vp, _i]),
     "df_kinfu_state_digest": (_i, [_vp, C.POINTER(C.c_ulonglong)]),
+    "df_kinfu_extract_mesh": (_i, [_vp, _i, _vp, _vp, _vp, _i, _vp, _i, C.POINTER(_i)]),
 }
 
 

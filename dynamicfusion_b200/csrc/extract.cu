@@ -11,6 +11,7 @@
 // needs nothing else -- on real scenes that is >90 % of them; only surface quads fetch the +x / +y / +z neighbours (L1/L2
 // hits).  Kernels: see the comment above extract_count_kernel.
 #include "df_common.cuh"
+#include <climits>
 
 using namespace dfb;
 
@@ -30,6 +31,24 @@ struct ExtractParams {
 
 __device__ __forceinline__ float vox_f(uint32_t v) { return half_bits_to_float((unsigned short)(v & 0xffffu)); }
 __device__ __forceinline__ bool sign_change(float F, float Fn) { return (F > 0 && Fn < 0) || (F < 0 && Fn > 0); }
+
+// centre of voxel (x, y, z) in volume coordinates
+__device__ __forceinline__ float3 voxel_centre(const ExtractParams &p, int x, int y, int z)
+{
+    return make_float3(((float)x + 0.5f) * p.vs.x, ((float)y + 0.5f) * p.vs.y, ((float)z + 0.5f) * p.vs.z);
+}
+
+// The point on the edge from voxel centre V (value F) to its +axis neighbour (value Fn), interpolated as tsdf_volume.cu:573-627 does,
+// then posed.  The one copy of the formula: the cloud's points and the mesh's vertices both come from here, so a mesh vertex on an edge
+// the cloud also emits is bit-identical to the cloud's point.
+__device__ __forceinline__ float3 edge_point(const ExtractParams &p, float3 V, float F, float Fn, int axis)
+{
+    const float d_inv = 1.f / (fabsf(F) + fabsf(Fn));
+    if (axis == 0) V.x = (V.x * fabsf(Fn) + (V.x + p.vs.x) * fabsf(F)) * d_inv;
+    else if (axis == 1) V.y = (V.y * fabsf(Fn) + (V.y + p.vs.y) * fabsf(F)) * d_inv;
+    else V.z = (V.z * fabsf(Fn) + (V.z + p.vs.z) * fabsf(F)) * d_inv;
+    return aff_mul(p.pose, V);
+}
 
 // Calls emit(point) for every zero crossing owned by this thread, in (voxel, axis) order.  tsdf_volume.cu:548-633.
 // the thread's own VX voxels (one 16-byte load when VX = 4); zeros past the end of the volume
@@ -67,38 +86,26 @@ __device__ __forceinline__ void thread_crossings(const ExtractParams &p, size_t 
         if (!vox_active(own[j])) continue;
         const int x = x0 + j;
         const float F = vox_f(own[j]);
-        const float3 V = make_float3(((float)x + 0.5f) * p.vs.x, ((float)y + 0.5f) * p.vs.y, ((float)z + 0.5f) * p.vs.z);
+        const float3 V = voxel_centre(p, x, y, z);
         if (x + 1 < p.Dx) {
             const uint32_t nv = (j + 1 < VX) ? own[(j + 1) % VX] : __ldg(p.data + v0 + VX);
             if (vox_active(nv)) {
                 const float Fn = vox_f(nv);
-                if (sign_change(F, Fn)) {
-                    const float Vnx = V.x + p.vs.x;
-                    const float d_inv = 1.f / (fabsf(F) + fabsf(Fn));
-                    emit(aff_mul(p.pose, make_float3((V.x * fabsf(Fn) + Vnx * fabsf(F)) * d_inv, V.y, V.z)));
-                }
+                if (sign_change(F, Fn)) emit(edge_point(p, V, F, Fn, 0));
             }
         }
         if (y + 1 < p.Dy) {
             const uint32_t nv = __ldg(p.data + v0 + j + p.Dx);
             if (vox_active(nv)) {
                 const float Fn = vox_f(nv);
-                if (sign_change(F, Fn)) {
-                    const float Vny = V.y + p.vs.y;
-                    const float d_inv = 1.f / (fabsf(F) + fabsf(Fn));
-                    emit(aff_mul(p.pose, make_float3(V.x, (V.y * fabsf(Fn) + Vny * fabsf(F)) * d_inv, V.z)));
-                }
+                if (sign_change(F, Fn)) emit(edge_point(p, V, F, Fn, 1));
             }
         }
         {
             const uint32_t nv = __ldg(p.data + v0 + j + slice);
             if (vox_active(nv)) {
                 const float Fn = vox_f(nv);
-                if (sign_change(F, Fn)) {
-                    const float Vnz = V.z + p.vs.z;
-                    const float d_inv = 1.f / (fabsf(F) + fabsf(Fn));
-                    emit(aff_mul(p.pose, make_float3(V.x, V.y, (V.z * fabsf(Fn) + Vnz * fabsf(F)) * d_inv)));
-                }
+                if (sign_change(F, Fn)) emit(edge_point(p, V, F, Fn, 2));
             }
         }
     }
@@ -302,6 +309,260 @@ extern "C" int df_extract_cloud_tracked(df_volume vol, df_aff3f pose, float *out
     DF_LAUNCH_CHECK();
     if (vx == 4) launch_pdl(extract_emit_kernel<4>, dim3(p.nblocks), dim3(EX_THREADS), 0, s, p, block_counts, offsets, super_off, (float4 *)out_points, capacity);
     else launch_pdl(extract_emit_kernel<1>, dim3(p.nblocks), dim3(EX_THREADS), 0, s, p, block_counts, offsets, super_off, (float4 *)out_points, capacity);
+    DF_LAUNCH_CHECK();
+    return 0;
+}
+
+// ------------------------------------------------------------------------------------------------------------------
+// Mesh extraction (marching cubes; the definition is in dfusion.h above df_extract_mesh).  Same block decomposition, quad loads,
+// activity skip and scans as the cloud: a counting pass writes two sets of block counts (vertices, triangles), each is scanned, then
+// one pass emits the vertices (ascending edge key) and one the triangles (ascending cell, table order).  A triangle finds its vertices
+// by binary search of their keys in the just-written edge_keys, inside the range of the block that owns the edge's lower endpoint.
+#define DF_MC_CONST static __device__ const
+#include "mc_table.h"
+
+namespace {
+
+__device__ __forceinline__ size_t vox_index(const ExtractParams &p, int x, int y, int z)
+{
+    return (size_t)x + (size_t)p.Dx * y + (size_t)p.Dx * p.Dy * z;
+}
+
+// case of the cell with min corner (x, y, z) -- bit i + 2j + 4k set iff corner (x+i, y+j, z+k) is inside (F < 0) -- or -1 if one of its
+// corners is inactive.  The caller keeps x < Dx-1, y < Dy-1, z < Dz-1.
+__device__ __forceinline__ int cell_case(const ExtractParams &p, int x, int y, int z)
+{
+    const size_t sy = (size_t)p.Dx, sz = (size_t)p.Dx * p.Dy;
+    const uint32_t *b = p.data + vox_index(p, x, y, z);
+    int c = 0;
+    bool active = true;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+        const uint32_t v = __ldg(b + (i & 1) + ((i & 2) ? sy : 0) + ((i & 4) ? sz : 0));
+        active &= vox_active(v);
+        c |= (int)vox_negative(v) << i;
+    }
+    return active ? c : -1;
+}
+
+// is one of the (up to four) cells around the edge from (x, y, z) along `axis` meshed?  Its endpoints differ in the inside test, so
+// every such cell has a mixed case and is meshed as soon as all its corners are active.
+__device__ __forceinline__ bool edge_has_meshed_cell(const ExtractParams &p, int x, int y, int z, int axis)
+{
+#pragma unroll
+    for (int j = 0; j < 2; ++j)
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+            const int cx = x - (axis == 0 ? 0 : j), cy = y - (axis == 1 ? 0 : (axis == 0 ? j : k)), cz = z - (axis == 2 ? 0 : k);
+            if (cx < 0 || cy < 0 || cz < 0 || cx >= p.Dx - 1 || cy >= p.Dy - 1 || cz >= p.Dz - 1) continue;
+            if (cell_case(p, cx, cy, cz) >= 0) return true;
+        }
+    return false;
+}
+
+// Calls emit(edge key, vertex) for every mesh vertex owned by this thread's quad (the edges leaving its voxels along +x, +y, +z), in
+// ascending key order.
+template <int VX, typename Emit>
+__device__ __forceinline__ void thread_mesh_vertices(const ExtractParams &p, size_t v0, const uint32_t (&own)[VX], Emit emit)
+{
+    bool any = false;
+#pragma unroll
+    for (int j = 0; j < VX; ++j) any |= vox_active(own[j]);
+    if (!any) return;
+    const size_t slice = (size_t)p.Dx * p.Dy;
+    const int z = (int)(v0 / slice);
+    const int rem = (int)(v0 - (size_t)z * slice);
+    const int y = rem / p.Dx;
+    const int x0 = rem - y * p.Dx;
+#pragma unroll
+    for (int j = 0; j < VX; ++j) {
+        if (!vox_active(own[j])) continue;
+        const int x = x0 + j;
+        const bool inside = vox_negative(own[j]);
+#pragma unroll
+        for (int axis = 0; axis < 3; ++axis) {
+            if (axis == 0 ? x + 1 >= p.Dx : axis == 1 ? y + 1 >= p.Dy : z + 1 >= p.Dz) continue;
+            const uint32_t nv = axis == 0 ? ((j + 1 < VX) ? own[(j + 1) % VX] : __ldg(p.data + v0 + VX))
+                                          : __ldg(p.data + v0 + j + (axis == 1 ? (size_t)p.Dx : slice));
+            if (!vox_active(nv) || vox_negative(nv) == inside) continue;
+            if (!edge_has_meshed_cell(p, x, y, z, axis)) continue;
+            emit(3u * (uint32_t)(v0 + j) + (uint32_t)axis, edge_point(p, voxel_centre(p, x, y, z), vox_f(own[j]), vox_f(nv), axis));
+        }
+    }
+}
+
+// Calls emit(voxel index, case) for every meshed cell whose min corner is one of this thread's voxels, in ascending order.
+template <int VX, typename Emit>
+__device__ __forceinline__ void thread_mesh_cells(const ExtractParams &p, size_t v0, const uint32_t (&own)[VX], Emit emit)
+{
+    bool any = false;
+#pragma unroll
+    for (int j = 0; j < VX; ++j) any |= vox_active(own[j]);
+    if (!any) return;
+    const size_t slice = (size_t)p.Dx * p.Dy;
+    const int z = (int)(v0 / slice);
+    if (z >= p.Dz - 1) return;
+    const int rem = (int)(v0 - (size_t)z * slice);
+    const int y = rem / p.Dx;
+    if (y >= p.Dy - 1) return;
+    const int x0 = rem - y * p.Dx;
+#pragma unroll
+    for (int j = 0; j < VX; ++j) {
+        if (!vox_active(own[j]) || x0 + j >= p.Dx - 1) continue;
+        const int c = cell_case(p, x0 + j, y, z);
+        if (c > 0 && c < 255) emit(v0 + j, c);
+    }
+}
+
+template <int VX>
+__device__ __forceinline__ void quad_mesh_counts(const ExtractParams &p, size_t v0, const uint32_t (&own)[VX], int &nv, int &nt)
+{
+    thread_mesh_vertices<VX>(p, v0, own, [&](uint32_t, float3) { ++nv; });
+    thread_mesh_cells<VX>(p, v0, own, [&](size_t, int c) { nt += df_mc_ntri[c]; });
+}
+
+template <int VX>
+__global__ void __launch_bounds__(EX_THREADS) mesh_count_kernel(const ExtractParams p, int *vblock_counts, int *tblock_counts)
+{
+    DF_PDL_ENTRY();
+    const size_t q0 = (size_t)blockIdx.x * EX_THREADS * EX_QPT;
+    uint32_t own[EX_QPT][VX];
+    load_block_quads<VX>(p, q0, own);
+    int nv = 0, nt = 0;
+#pragma unroll
+    for (int i = 0; i < EX_QPT; ++i) quad_mesh_counts<VX>(p, (q0 + (size_t)(i * EX_THREADS) + threadIdx.x) * VX, own[i], nv, nt);
+    if (!__syncthreads_or(nv | nt)) {
+        if (threadIdx.x == 0) { vblock_counts[blockIdx.x] = 0; tblock_counts[blockIdx.x] = 0; }
+        return;
+    }
+    int vtotal, ttotal;
+    block_exclusive_scan(nv, &vtotal);
+    block_exclusive_scan(nt, &ttotal);
+    if (threadIdx.x == 0) { vblock_counts[blockIdx.x] = vtotal; tblock_counts[blockIdx.x] = ttotal; }
+}
+
+template <int VX>
+__global__ void __launch_bounds__(EX_THREADS) mesh_vertex_emit_kernel(const ExtractParams p, const int *block_counts, const int *offsets,
+                                                                      const int *super_off, float4 *vertices, uint32_t *keys, int vcap)
+{
+    DF_PDL_ENTRY();
+    if (block_counts[blockIdx.x] == 0) return;
+    const size_t q0 = (size_t)blockIdx.x * EX_THREADS * EX_QPT;
+    uint32_t own[EX_QPT][VX];
+    load_block_quads<VX>(p, q0, own);
+    int run = super_off[blockIdx.x >> 10] + offsets[blockIdx.x];
+#pragma unroll
+    for (int i = 0; i < EX_QPT; ++i) {
+        const size_t v0 = (q0 + (size_t)(i * EX_THREADS) + threadIdx.x) * VX;
+        int c = 0;
+        thread_mesh_vertices<VX>(p, v0, own[i], [&](uint32_t, float3) { ++c; });
+        int total;
+        int k = run + block_exclusive_scan(c, &total);
+        if (c)
+            thread_mesh_vertices<VX>(p, v0, own[i], [&](uint32_t key, float3 q) {
+                if (k < vcap) { vertices[k] = make_float4(q.x, q.y, q.z, 0.f); keys[k] = key; }
+                ++k;
+            });
+        run += total;
+    }
+}
+
+// index of the vertex with edge key `key`: binary search in the range of the block that owns the key's voxel
+template <int VX>
+__device__ __forceinline__ int find_vertex(const uint32_t *keys, uint32_t key, const int *block_counts, const int *offsets, const int *super_off)
+{
+    const int blk = (int)((key / 3u) / VX / (EX_THREADS * EX_QPT));
+    int lo = super_off[blk >> 10] + offsets[blk], hi = lo + block_counts[blk];
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (keys[mid] < key) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
+
+template <int VX>
+__global__ void __launch_bounds__(EX_THREADS) mesh_triangle_emit_kernel(const ExtractParams p, const int *vblock_counts, const int *voffsets,
+                                                                        const int *vsuper_off, const uint32_t *keys, const int *counts, int vcap,
+                                                                        const int *block_counts, const int *offsets, const int *super_off,
+                                                                        int3 *triangles, int tcap)
+{
+    DF_PDL_ENTRY();
+    if (block_counts[blockIdx.x] == 0 || counts[0] > vcap) return;    // vertex overflow: the indices cannot be resolved
+    const size_t q0 = (size_t)blockIdx.x * EX_THREADS * EX_QPT;
+    uint32_t own[EX_QPT][VX];
+    load_block_quads<VX>(p, q0, own);
+    const uint32_t sy = (uint32_t)p.Dx, sz = (uint32_t)p.Dx * (uint32_t)p.Dy;
+    int run = super_off[blockIdx.x >> 10] + offsets[blockIdx.x];
+#pragma unroll
+    for (int i = 0; i < EX_QPT; ++i) {
+        const size_t v0 = (q0 + (size_t)(i * EX_THREADS) + threadIdx.x) * VX;
+        int c = 0;
+        thread_mesh_cells<VX>(p, v0, own[i], [&](size_t, int cs) { c += df_mc_ntri[cs]; });
+        int total;
+        int k = run + block_exclusive_scan(c, &total);
+        if (c)
+            thread_mesh_cells<VX>(p, v0, own[i], [&](size_t v, int cs) {
+                const int n = df_mc_ntri[cs];
+                for (int t = 0; t < n; ++t, ++k) {
+                    if (k >= tcap) continue;
+                    int idx[3];
+#pragma unroll
+                    for (int q = 0; q < 3; ++q) {
+                        const signed char *e = df_mc_edges[df_mc_tris[cs][3 * t + q]];
+                        const uint32_t owner = (uint32_t)v + (uint32_t)e[0] + sy * (uint32_t)e[1] + sz * (uint32_t)e[2];
+                        idx[q] = find_vertex<VX>(keys, 3u * owner + (uint32_t)e[3], vblock_counts, voffsets, vsuper_off);
+                    }
+                    triangles[k] = make_int3(idx[0], idx[1], idx[2]);
+                }
+            });
+        run += total;
+    }
+}
+
+}  // namespace
+
+extern "C" size_t df_extract_mesh_workspace_bytes(df_volume vol)
+{
+    return 2 * df_extract_workspace_bytes(vol);          // one set of block counts / offsets / super sums for vertices, one for triangles
+}
+
+extern "C" int df_extract_mesh(df_volume vol, df_aff3f pose, const unsigned char *activity, float *vertices, uint32_t *edge_keys, int vcap,
+                               int32_t *triangles, int tcap, int *counts_dev, void *workspace, void *stream)
+{
+    if (vcap < 0 || tcap < 0 || !counts_dev || !workspace) return (int)cudaErrorInvalidValue;
+    const int vx = pick_vx(vol);
+    ExtractParams p = make_params(vol, pose, vx);
+    p.activity = activity;
+    const int nsuper = (p.nblocks + 1023) / 1024;
+    if (nsuper > 1024) return (int)cudaErrorInvalidValue;               // > 2^20 blocks (volume > 1024^3 voxels)
+    int *vcounts = (int *)workspace, *voff = vcounts + p.nblocks, *vsuper_tot = voff + p.nblocks, *vsuper_off = vsuper_tot + 1024;
+    int *tcounts = (int *)workspace + df_extract_workspace_bytes(vol) / sizeof(int);
+    int *toff = tcounts + p.nblocks, *tsuper_tot = toff + p.nblocks, *tsuper_off = tsuper_tot + 1024;
+    cudaStream_t s = (cudaStream_t)stream;
+    const dim3 grid(p.nblocks), block(EX_THREADS);
+    if (vx == 4) launch_pdl(mesh_count_kernel<4>, grid, block, 0, s, p, vcounts, tcounts);
+    else launch_pdl(mesh_count_kernel<1>, grid, block, 0, s, p, vcounts, tcounts);
+    DF_LAUNCH_CHECK();
+    // the scans report the true totals (capacity INT_MAX); the emit passes clamp
+    launch_pdl(extract_scan_local_kernel, dim3(nsuper), dim3(1024), 0, s, (const int *)vcounts, voff, p.nblocks, vsuper_tot);
+    launch_pdl(extract_scan_super_kernel, dim3(1), dim3(1024), 0, s, (const int *)vsuper_tot, nsuper, vsuper_off, INT_MAX, counts_dev);
+    launch_pdl(extract_scan_local_kernel, dim3(nsuper), dim3(1024), 0, s, (const int *)tcounts, toff, p.nblocks, tsuper_tot);
+    launch_pdl(extract_scan_super_kernel, dim3(1), dim3(1024), 0, s, (const int *)tsuper_tot, nsuper, tsuper_off, INT_MAX, counts_dev + 1);
+    DF_LAUNCH_CHECK();
+    if (vx == 4) {
+        launch_pdl(mesh_vertex_emit_kernel<4>, grid, block, 0, s, p, (const int *)vcounts, (const int *)voff, (const int *)vsuper_off,
+                   (float4 *)vertices, edge_keys, vcap);
+        launch_pdl(mesh_triangle_emit_kernel<4>, grid, block, 0, s, p, (const int *)vcounts, (const int *)voff, (const int *)vsuper_off,
+                   (const uint32_t *)edge_keys, (const int *)counts_dev, vcap, (const int *)tcounts, (const int *)toff, (const int *)tsuper_off,
+                   (int3 *)triangles, tcap);
+    } else {
+        launch_pdl(mesh_vertex_emit_kernel<1>, grid, block, 0, s, p, (const int *)vcounts, (const int *)voff, (const int *)vsuper_off,
+                   (float4 *)vertices, edge_keys, vcap);
+        launch_pdl(mesh_triangle_emit_kernel<1>, grid, block, 0, s, p, (const int *)vcounts, (const int *)voff, (const int *)vsuper_off,
+                   (const uint32_t *)edge_keys, (const int *)counts_dev, vcap, (const int *)tcounts, (const int *)toff, (const int *)tsuper_off,
+                   (int3 *)triangles, tcap);
+    }
     DF_LAUNCH_CHECK();
     return 0;
 }

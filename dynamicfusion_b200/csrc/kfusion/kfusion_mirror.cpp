@@ -432,6 +432,22 @@ void TsdfVolume::fetchNormals(const DeviceArray<Point>& cloud, DeviceArray<Norma
                                   Rinv.val, gradient_delta_factor_, (float *)normals.ptr(), 0));
     cudaSafeCall(cudaDeviceSynchronize());
 }
+void TsdfVolume::fetchMesh(DeviceArray<Point>& vertices, DeviceArray<Normal>& normals, DeviceArray<int>& triangles) const
+{
+    const df_volume v = vol_of(data_, dims_, getVoxelSize(), trunc_dist_, max_weight_);
+    DeviceMemory ws(df_extract_mesh_workspace_bytes(v)), counts(64), keys;
+    for (;;) {     // the counts are the true totals: a second call with the arrays resized to them fits exactly
+        keys.create(std::max<size_t>(vertices.size(), 1) * sizeof(uint32_t));
+        dfSafeCall(df_extract_mesh(v, to_df(pose_), activity_, (float *)vertices.ptr(), keys.ptr<uint32_t>(), (int)vertices.size(), triangles.ptr(),
+                                   (int)(triangles.size() / 3), counts.ptr<int>(), ws.ptr<void>(), 0));
+        int c[2];
+        cudaSafeCall(cudaMemcpy(c, counts.ptr<int>(), sizeof c, cudaMemcpyDeviceToHost));
+        if ((size_t)c[0] == vertices.size() && (size_t)c[1] * 3 == triangles.size()) break;
+        if (c[0]) vertices.create(c[0]); else vertices.release();
+        if (c[1]) triangles.create((size_t)c[1] * 3); else triangles.release();
+    }
+    fetchNormals(vertices, normals);
+}
 void TsdfVolume::compute_points()
 {
     *cloud_ = fetchCloud(*cloud_buffer_);
@@ -890,6 +906,26 @@ bool KinFu::operator()(const cuda::Depth& depth, const cuda::Image& /*image*/)
         warp_->adoptDeviceNodes(nodes, 0, (int)info[1]);
     }
     return r == 1;
+}
+void KinFu::getMesh(cv::Mat& vertices, cv::Mat& normals, cv::Mat& triangles, bool live) const
+{
+    int vcap = std::max(params_.volume_dims[0] * params_.volume_dims[1] * 4, 1024), tcap = 2 * vcap, c[2] = {0, 0};
+    for (;;) {     // the counts are the true totals: one more call with buffers of that size fits
+        DeviceMemory v((size_t)vcap * 16), n((size_t)vcap * 16), keys((size_t)vcap * 4), t((size_t)tcap * 12);
+        const int st = df_kinfu_extract_mesh(handle_, live ? DF_MESH_LIVE : 0, v.ptr<float>(), n.ptr<float>(), keys.ptr<uint32_t>(), vcap,
+                                             t.ptr<int32_t>(), tcap, c);
+        if (st) kfusion::cuda::error(df_error_string(st), __FILE__, __LINE__);
+        if (c[0] <= vcap && c[1] <= tcap) {
+            vertices.create(1, c[0], CV_32FC4); normals.create(1, c[0], CV_32FC4); triangles.create(c[1], 1, CV_32SC3);
+            if (c[0]) {
+                cudaSafeCall(cudaMemcpy(vertices.ptr<float>(), v.ptr<float>(), (size_t)c[0] * 16, cudaMemcpyDeviceToHost));
+                cudaSafeCall(cudaMemcpy(normals.ptr<float>(), n.ptr<float>(), (size_t)c[0] * 16, cudaMemcpyDeviceToHost));
+            }
+            if (c[1]) cudaSafeCall(cudaMemcpy(triangles.ptr<int>(), t.ptr<int32_t>(), (size_t)c[1] * 12, cudaMemcpyDeviceToHost));
+            return;
+        }
+        vcap = std::max(vcap, c[0]); tcap = std::max(tcap, c[1]);
+    }
 }
 void KinFu::dynamicfusion(cuda::Depth& depth, cuda::Cloud live_frame, cuda::Normals /*current_normals*/)
 {

@@ -43,6 +43,7 @@ struct KinFu {
     void *integrate_ws = nullptr;
     void *extend_ws = nullptr; int *M_dev = nullptr;   // df_extend_field workspace / new node count (DF_KINFU_EXTEND_FIELD)
     void *fusion_ws = nullptr;             // df_integrate_warped workspace (DF_KINFU_WARPED_INTEGRATE)
+    void *mesh_ws = nullptr; size_t mesh_ws_bytes = 0;   // df_kinfu_extract_mesh: workspace, counts, scratch normals (allocated on first use)
     unsigned char *activity = nullptr; size_t activity_bytes = 0;   // dfusion.h DF_ACTIVITY_VOXELS: which stretches of the volume hold surface
     float *pinned = nullptr;             // 16 floats: T(12) + ok
     std::vector<float> poses;            // 12 floats per pose
@@ -668,7 +669,7 @@ extern "C" void df_kinfu_destroy(void *h)
     cudaFree(k->cloud); cudaFree(k->cloud_nrm); cudaFree(k->cloud_count); cudaFree(k->nodes); cudaFree(k->node_grid);
     cudaFree(k->icp_T); cudaFree(k->icp_ok); cudaFree(k->icp_scratch); cudaFree(k->solve_ws); cudaFree(k->solve_stats);
     cudaFree(k->f2_ws); cudaFree(k->f2_stats);
-    cudaFree(k->extract_ws); cudaFree(k->project_ws); cudaFree(k->activity); cudaFree(k->integrate_ws); cudaFree(k->fusion_ws); cudaFree(k->extend_ws); cudaFree(k->M_dev); cudaFreeHost(k->pinned); cudaFree(k->n_upd);
+    cudaFree(k->extract_ws); cudaFree(k->project_ws); cudaFree(k->activity); cudaFree(k->integrate_ws); cudaFree(k->fusion_ws); cudaFree(k->mesh_ws); cudaFree(k->extend_ws); cudaFree(k->M_dev); cudaFreeHost(k->pinned); cudaFree(k->n_upd);
     for (int e = 0; e <= NSTAGES; ++e) if (k->ev[e]) cudaEventDestroy(k->ev[e]);
     delete k;
 }
@@ -880,4 +881,49 @@ extern "C" int df_kinfu_get_stage_ms(void *h, float *ms, int n)
     const int m = n < NSTAGES ? n : NSTAGES;
     for (int i = 0; i < m; ++i) ms[i] = k->stage_ms[i];
     return m;
+}
+
+// Mesh of the current model, on demand.  It only reads the volume and the activity map, on the main stream after the last integrate; it
+// neither launches nor waits for the deferred extraction (which only reads the volume as well) and writes nothing the loop owns.
+extern "C" int df_kinfu_extract_mesh(void *h, int flags, float *vertices, float *normals, uint32_t *edge_keys, int vcap,
+                                     int32_t *triangles, int tcap, int *counts_host)
+{
+    KinFu *k = (KinFu *)h;
+    if (!k || !counts_host || vcap < 0 || tcap < 0) return (int)cudaErrorInvalidValue;
+    const bool live = (flags & DF_MESH_LIVE) != 0;
+    if (live && ((k->p.flags & DF_KINFU_RIGID_ONLY) || k->M < 8)) return (int)cudaErrorInvalidValue;   // no field the loop would warp with
+    cudaSetDevice(k->device);
+    cudaStream_t s = k->stream;
+    const df_volume vol = vol_of(*k);
+    const size_t ws_bytes = df_extract_mesh_workspace_bytes(vol);
+    const bool scratch_normals = live && !normals;     // the warp needs normals: a vertex with a NaN normal is left in place
+    const size_t need = ws_bytes + 256 + (scratch_normals ? (size_t)vcap * 16 : 0);
+    if (need > k->mesh_ws_bytes) {
+        cudaFree(k->mesh_ws);
+        k->mesh_ws = nullptr; k->mesh_ws_bytes = 0;
+        if (cudaMalloc(&k->mesh_ws, need) != cudaSuccess) return (int)cudaGetLastError();
+        k->mesh_ws_bytes = need;
+    }
+    int *counts_dev = (int *)((char *)k->mesh_ws + ws_bytes);
+    float *nrm = scratch_normals ? (float *)((char *)k->mesh_ws + ws_bytes + 256) : normals;
+    const df_kinfu_params &p = k->p;
+    if (int st = df_extract_mesh(vol, p.volume_pose, k->activity, vertices, edge_keys, vcap, triangles, tcap, counts_dev, k->mesh_ws, s)) return st;
+    if (nrm) {
+        float vol_pose[12], Rinv_vol[9];
+        memcpy(vol_pose, p.volume_pose.R, 36); memcpy(vol_pose + 9, p.volume_pose.t, 12);
+        dfh_mat3_inv(vol_pose, Rinv_vol);
+        if (int st = df_extract_normals(vol, vertices, vcap, counts_dev, p.volume_pose, Rinv_vol, p.gradient_delta_factor, nrm, s)) return st;
+    }
+    int counts[2] = {0, 0};
+    if (cudaMemcpyAsync(counts, counts_dev, sizeof counts, cudaMemcpyDeviceToHost, s) != cudaSuccess || cudaStreamSynchronize(s) != cudaSuccess)
+        return (int)cudaGetLastError();
+    counts_host[0] = counts[0]; counts_host[1] = counts[1];
+    if (live) {
+        const int n = counts[0] < vcap ? counts[0] : vcap;
+        float id12[12];
+        dfh_aff_identity(id12);
+        if (int st = df_warp(k->nodes, k->M, k->node_grid, vertices, nrm, n, 4, to_aff(id12), DF_WARP_NORMAL_ROTATE_ONLY, nullptr, nullptr, s)) return st;
+        if (cudaStreamSynchronize(s) != cudaSuccess) return (int)cudaGetLastError();
+    }
+    return 0;
 }

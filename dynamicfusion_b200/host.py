@@ -101,27 +101,38 @@ def resizePointsNormals(points: torch.Tensor, normals: torch.Tensor):
     return vd, nd
 
 
-def save_ply(path, points, normals=None) -> int:
+def save_ply(path, points, normals=None, triangles=None) -> int:
     """Export of the extracted canonical cloud (SURVEY 8f(4); Report.md "Export the reconstructions to .ply"): the Python twin of
     kfusion::writePly (include/kfusion/io/ply.hpp) -- binary little-endian PLY, float x y z [nx ny nz]; points with a NaN coordinate
-    are skipped, NaN normals written as 0.  points / normals: host or device arrays of shape [N, >=3]."""
-    pts = points.detach().cpu().numpy() if isinstance(points, torch.Tensor) else np.asarray(points)
-    pts = np.asarray(pts, np.float32)[:, :3]
-    keep = ~np.isnan(pts).any(1)
+    are skipped, NaN normals written as 0.  points / normals: host or device arrays of shape [N, >=3].
+    triangles ([M, 3] int32 vertex indices, e.g. from TsdfVolume.fetchMesh / KinFu.mesh): the mesh form, which adds `element face M`
+    (`property list uchar int vertex_indices`) and writes every vertex as given -- mesh vertices are finite, and dropping one would shift
+    the indices.  Returns the number of vertices written."""
+    host = lambda a: np.asarray(a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else a)
+    pts = np.asarray(host(points), np.float32)[:, :3]
+    keep = ~np.isnan(pts).any(1) if triangles is None else np.ones(len(pts), bool)
     cols = [pts[keep]]
     if normals is not None:
-        nrm = normals.detach().cpu().numpy() if isinstance(normals, torch.Tensor) else np.asarray(normals)
-        nrm = np.asarray(nrm, np.float32)[:, :3][keep].copy()
+        nrm = np.asarray(host(normals), np.float32)[:, :3][keep].copy()
         nrm[np.isnan(nrm).any(1)] = 0.0
         cols.append(nrm)
     data = np.ascontiguousarray(np.concatenate(cols, 1), "<f4")
     with open(path, "wb") as f:
-        f.write(b"ply\nformat binary_little_endian 1.0\ncomment dynamicfusion canonical cloud\n")
+        what = b"canonical cloud" if triangles is None else b"mesh"
+        f.write(b"ply\nformat binary_little_endian 1.0\ncomment dynamicfusion " + what + b"\n")
         f.write(f"element vertex {len(data)}\nproperty float x\nproperty float y\nproperty float z\n".encode())
         if normals is not None:
             f.write(b"property float nx\nproperty float ny\nproperty float nz\n")
+        if triangles is not None:
+            tri = np.asarray(host(triangles), np.int32).reshape(-1, 3)
+            f.write(f"element face {len(tri)}\nproperty list uchar int vertex_indices\n".encode())
         f.write(b"end_header\n")
         f.write(data.tobytes())
+        if triangles is not None:
+            faces = np.empty(len(tri), np.dtype([("n", "u1"), ("i", "<i4", 3)]))
+            faces["n"] = 3
+            faces["i"] = tri
+            f.write(faces.tobytes())
     return len(data)
 
 
@@ -150,6 +161,7 @@ class TsdfVolume:
         self.raycast_step_factor_ = 0.75
         self.cloud_capacity = 0
         self._ws = None
+        self._mesh_ws = None
         self._proj_ws = None
         self.create(dims)
 
@@ -296,6 +308,24 @@ class TsdfVolume:
                                                    self._ws.data_ptr(), self.activity_.data_ptr() if self.activity_ is not None else None,
                                                    _stream()))
         return out, count
+
+    def fetchMesh(self, vcap: int, tcap: int, normals: bool = True):
+        """Triangle mesh of the zero level set (dfusion.h df_extract_mesh; marching cubes), through the activity map when the volume
+        tracks one.  Returns device tensors (vertices [vcap, 4] float32, normals [vcap, 4] or None, edge keys [vcap] int32 holding the u32
+        keys, triangles [tcap, 3] int32, counts [2] int32 = true vertex / triangle totals) -- no host sync.  Only the first
+        min(count, cap) rows are written, and no triangle is when the vertices overflow."""
+        need = _lib().df_extract_mesh_workspace_bytes(self._vol())
+        if self._mesh_ws is None or self._mesh_ws.numel() < need:
+            self._mesh_ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        verts = torch.empty((max(vcap, 1), 4), dtype=torch.float32, device=self.device)
+        keys = torch.empty(max(vcap, 1), dtype=torch.int32, device=self.device)
+        tris = torch.empty((max(tcap, 1), 3), dtype=torch.int32, device=self.device)
+        counts = torch.zeros(2, dtype=torch.int32, device=self.device)
+        capi.check(_lib().df_extract_mesh(self._vol(), capi.make_aff(*self.pose_), self.activity_.data_ptr() if self.activity_ is not None else None,
+                                          verts.data_ptr(), keys.data_ptr(), vcap, tris.data_ptr(), tcap, counts.data_ptr(),
+                                          self._mesh_ws.data_ptr(), _stream()))
+        nrm = self.fetchNormals(verts, vcap, counts[:1]) if normals and vcap > 0 else None
+        return verts[:vcap], nrm, keys[:vcap], tris[:tcap], counts
 
     def fetchNormals(self, cloud: torch.Tensor, n: int, count_dev: torch.Tensor | None = None):
         Rinv = np.linalg.inv(self.pose_[0].astype(np.float64)).astype(np.float32)

@@ -21,6 +21,7 @@ EXTEND_FIELD = 16         # DF_KINFU_EXTEND_FIELD: grow the warp field over unsu
 F2_SOLVE = 32             # DF_KINFU_F2_SOLVE: robust 6-DoF data term + regulariser instead of the translation-only solve (SURVEY 8f(2))
 USE_DEPTH = 64            # DF_KINFU_USE_DEPTH: the reference's compile-time USE_DEPTH frame loop (depth-pyramid ICP)
 WARPED_INTEGRATE = 8      # DF_KINFU_WARPED_INTEGRATE: per-voxel warped fusion (SURVEY 8f(1)) instead of the rigid fallback
+MESH_LIVE = 1             # DF_MESH_LIVE: df_kinfu_extract_mesh carries the mesh through the current warp field
 
 
 class KinFuParams:
@@ -119,6 +120,27 @@ class KinFu:
         v = (C.c_ulonglong * 4)()
         capi.check(self.lib.df_kinfu_state_digest(self.h, v))
         return [int(x) for x in v]
+
+    def mesh(self, live: bool = False, normals: bool = True):
+        """The current model as a triangle mesh (df_kinfu_extract_mesh): canonical, or carried into the live frame through the warp field
+        (live=True; a rigid-only object, or one whose field does not exist yet, raises).  Leaves the object's state untouched.  Returns
+        numpy (vertices [n, 3] float32, normals [n, 3] float32 or None, triangles [m, 3] int32, edge keys [n] uint32)."""
+        vcap = max(int(self.params.cloud_capacity), 1024)
+        tcap = 2 * vcap
+        counts = (C.c_int * 2)()
+        while True:
+            v = torch.empty((vcap, 4), dtype=torch.float32, device="cuda")
+            n = torch.empty((vcap, 4), dtype=torch.float32, device="cuda") if normals else None
+            k = torch.empty(vcap, dtype=torch.int32, device="cuda")
+            t = torch.empty((tcap, 3), dtype=torch.int32, device="cuda")
+            capi.check(self.lib.df_kinfu_extract_mesh(self.h, MESH_LIVE if live else 0, v.data_ptr(), n.data_ptr() if normals else None,
+                                                      k.data_ptr(), vcap, t.data_ptr(), tcap, counts))
+            if counts[0] <= vcap and counts[1] <= tcap:
+                break
+            vcap, tcap = max(vcap, counts[0]), max(tcap, counts[1])     # the counts are true totals: one more call fits
+        nv, nt = counts[0], counts[1]
+        return (v[:nv, :3].cpu().numpy(), n[:nv, :3].cpu().numpy() if normals else None, t[:nt].cpu().numpy(),
+                k[:nv].cpu().numpy().view(np.uint32))
 
     def stage_ms(self) -> dict:
         v = (C.c_float * 10)()

@@ -16,11 +16,13 @@
 
 #define CV_8U 0
 #define CV_16U 2
+#define CV_32S 4
 #define CV_32F 5
 #define CV_MAKETYPE(depth, cn) ((depth) + (((cn) - 1) << 3))
 #define CV_8UC4 CV_MAKETYPE(CV_8U, 4)
 #define CV_32FC3 CV_MAKETYPE(CV_32F, 3)
 #define CV_32FC4 CV_MAKETYPE(CV_32F, 4)
+#define CV_32SC3 CV_MAKETYPE(CV_32S, 3)
 #define CV_Assert(expr)                                                                       \
     do {                                                                                      \
         if (!(expr)) { std::fprintf(stderr, "CV_Assert failed: %s (%s:%d)\n", #expr, __FILE__, __LINE__); std::abort(); } \

@@ -133,6 +133,30 @@ int df_extract_cloud_tracked(df_volume vol, df_aff3f pose, float *out_points, in
 int df_extract_normals(df_volume vol, const float *points, int n_points, const int *count_dev, df_aff3f pose,
                        const float *Rinv_host9, float delta_factor, float *out_normals, void *stream);
 
+/* Triangle mesh of the volume's zero level set (marching cubes; not in the reference, whose next steps ask for a .ply / .obj export,
+ * Report.md:57).  Definition -- in the volume's own conventions, so that it agrees with the cloud:
+ *   a voxel is ACTIVE iff W != 0 && F != 1 (as for the cloud); a corner is INSIDE iff F < 0 (-0 is not inside);
+ *   cell (x, y, z), x < Dx-1, y < Dy-1, z < Dz-1, has the 8 corners (x+i, y+j, z+k); it is MESHED iff all 8 are active and its inside
+ *   mask is neither 0 nor 255;
+ *   one VERTEX per voxel edge (v, axis) (axis 0/1/2 = +x/+y/+z) whose endpoints differ in the inside test and which borders at least one
+ *   meshed cell; its edge key is 3*v + axis (v = linear voxel index; fits in 32 bits up to 1024^3 voxels); vertices come out in
+ *   ascending key order; the position is the cloud's interpolation of that edge, posed by `pose` -- the same device code, so a vertex on an
+ *   edge the cloud also emits (strict sign change, both endpoints active) is bit-identical to that cloud point;
+ *   TRIANGLES (int32[3] indices into the vertices): every meshed cell in ascending cell index emits the triangles of its case in the order
+ *   of the generated table (csrc/mc_table.h, tools/gen_mc_table.py), counter-clockwise seen from the outside (F > 0), so the face normal
+ *   points along the TSDF gradient as df_extract_normals does.  Each cube face is decided from its own four signs (an ambiguous face
+ *   separates its inside corners), so neighbouring cells agree and the mesh has no cracks.
+ * Deterministic (no atomics decide order or content).  Every crossing edge's lower endpoint and every meshed cell's min corner is active,
+ * so the activity map (as df_extract_cloud_tracked; NULL = full scan) returns exactly the full scan's mesh.  Vertices are found by binary
+ * search of their keys -- no per-voxel index array.
+ * counts_dev (device, 2 x int32): [0] vertices, [1] triangles -- the TRUE totals, never clamped.  Vertices beyond vcap and triangles
+ * beyond tcap are not written; if the vertices overflow, no triangle is written (their indices would be unresolvable).
+ * workspace: df_extract_mesh_workspace_bytes() bytes. */
+size_t df_extract_mesh_workspace_bytes(df_volume vol);
+int df_extract_mesh(df_volume vol, df_aff3f pose, const unsigned char *activity,
+                    float *vertices /* float4, w = 0 */, uint32_t *edge_keys, int vcap,
+                    int32_t *triangles /* [tcap][3] */, int tcap, int *counts_dev, void *workspace, void *stream);
+
 /* ------------------------------------------------------------------ image processing ----------------------------------------------------- */
 /* device::bilateralFilter (internal.hpp:125, imgproc.cu:11-57) */
 int df_bilateral(const uint16_t *src, size_t src_pitch, int cols, int rows, uint16_t *dst, size_t dst_pitch,
@@ -408,6 +432,17 @@ int df_kinfu_state_digest(void *kinfu, unsigned long long *out4_host);
 /* per-stage milliseconds of the last frame (DF_KINFU_STAGE_TIMING): preprocess, icp, raycast_canonical, warp1, solve,
  * warp2, project_remove, integrate, extract, raycast_prev; returns the number written */
 int df_kinfu_get_stage_ms(void *kinfu, float *ms_host, int n);
+
+/* The frame loop's current model as a mesh (df_extract_mesh of its volume at the volume pose, through its activity map), on the object's
+ * stream, ordered after its last integrate.  Synchronous; counts_host[2] as df_extract_mesh's counts.  normals (optional, float4):
+ * df_extract_normals at the vertices.  DF_MESH_LIVE: vertices (and normals, rotation only) are carried through the current warp field by
+ * df_warp with warp_to_live = identity, as the loop warps its canonical points -- a vertex whose normal is NaN (within two voxels of the
+ * volume's border) stays where it is, as df_warp leaves such points; an object without warp nodes (rigid-only, or before the field exists)
+ * returns cudaErrorInvalidValue.  Runs on demand, never inside df_kinfu_process_*: the object's state (volume, cloud, nodes, poses, the
+ * pending extraction on its auxiliary stream) is left exactly as it was.  The workspace is allocated on first use, not at create. */
+#define DF_MESH_LIVE 1
+int df_kinfu_extract_mesh(void *kinfu, int flags, float *vertices, float *normals, uint32_t *edge_keys, int vcap,
+                          int32_t *triangles, int tcap, int *counts_host);
 
 #ifdef __cplusplus
 }

@@ -56,6 +56,9 @@ namespace kfusion
             void swap(CudaData& data);
             DeviceArray<Point> fetchCloud(DeviceArray<Point>& cloud_buffer) const;
             void fetchNormals(const DeviceArray<Point>& cloud, DeviceArray<Normal>& normals) const;
+            // not in the reference: the triangle mesh of the zero level set (dfusion.h df_extract_mesh, marching cubes) at the volume pose; the
+            // arrays are resized to the mesh (triangles: 3 vertex indices each), normals as fetchNormals computes them at the vertices
+            void fetchMesh(DeviceArray<Point>& vertices, DeviceArray<Normal>& normals, DeviceArray<int>& triangles) const;
             void compute_points();
             void compute_normals();
 

@@ -69,6 +69,10 @@ namespace kfusion
         void dynamicfusion(cuda::Depth& depth, cuda::Cloud live_frame, cuda::Normals current_normals);
         void renderImage(cuda::Image& image, const Affine3f& pose, int flags = 0);
         Affine3f getCameraPose (int time = -1) const;
+        // not in the reference: the current model as a host mesh (df_kinfu_extract_mesh) -- vertices / normals 1 x N CV_32FC4, triangles
+        // M x 1 CV_32SC3; live = true carries it through the warp field into the live frame.  kfusion::writePly(path, vertices, normals,
+        // triangles) exports it.
+        void getMesh(cv::Mat& vertices, cv::Mat& normals, cv::Mat& triangles, bool live = false) const;
     private:
         void allocate_buffers();
 
